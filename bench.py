@@ -3,19 +3,23 @@
 RANSAC SE(3)) on B200, BASELINE.json config C2: a batch of 256 synthetic frame pairs, 1000 ORB keypoints
 per frame, per GPU.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
          bench.py --gpus N --steps K --warmup W
 
 One "step" = Node::matchNodePair (node.cpp:1305) for every pair of the batch through the C ABI.
   value : pairs/s with the nodes' features already resident in HBM (rgbdslam_b200_match_pairs on node
-          handles), CUDA-event timed, L2 flushed between steps, max over ranks.
+          handles) over exactly K timed steps in steady state (the pipeline is full when the timed region
+          starts and when it ends), max over ranks.
   e2e   : same metric through rgbdslam_b200_match_pairs_host with pinned HOST buffers in and HOST
           MatchingResults out (H2D + D2H inside the timed region).
   roofline     : the Hamming kernel against the HBM roofline (SURVEY.md 8d: 72 000 B / pair @1000 kp).
   cpu_baseline : the CPU oracle (plain-C port of the reference path) on this box's host cores.
 --impl reference times that CPU oracle as the reference arm (the reference itself cannot be built: ROS /
 Qt / PCL / g2o / OpenCV-C++ are absent -- see DESIGN.md).
+--dump-outputs DIR writes what the last timed step of both paths returned to its caller (rank 0), one
+DIR/<path>_<array>_<field>.npy per field, integers as float64: the inputs are fixed by seeds, so two builds
+of the library can be compared output for output.
 """
 from __future__ import annotations
 
@@ -43,7 +47,7 @@ ALGO_BYTES_PER_PAIR = (N_KP + N_KP) * 32 + N_KP * 8  # SURVEY.md section 8(d): 7
 # one string for both arms (the driver compares config.workload of `ours` and `reference`)
 WORKLOAD = (f"C2: {PAIRS_PER_GPU} frame pairs x {N_KP} ORB kp per GPU, Hamming BF match + 4-pt RANSAC "
             "(200 hypotheses, max_matches 300), synthetic feature-level pairs (rgbdslam_v2_b200/synth.py make_batch)")
-MIN_TIMED_MS = 50.0  # the timed regions cover at least this much device time whatever --steps says
+MIN_TIMED_MS = 50.0  # the rendered-frame C2 sub-measurement times at least this much
 
 
 def measured_peaks():
@@ -698,30 +702,58 @@ def run_ours(args, rank, local_rank, world):
                              bb["n_older"], bb["id_newer"], bb["id_older"], (st["res"], st["allm"], st["inl"]), seed=SEED,
                              first_pair_index=st["first"])
 
-    def finish(k):
-        """results of step k are on the host; N > 1: kept for the exchange at the end of the region"""
+    def finish(k, timed):
+        """results of step k are on the host; N > 1: a timed step's are kept for the exchange at the end of the region"""
         fe.wait_slot(1 + k % DEPTH)
-        if comm is not None:
+        if comm is not None and timed:
             n = local_edges["n"]
             local_edges["buf"][n:n + PAIRS_PER_GPU] = sets[k % DEPTH]["res"]
             local_edges["n"] = n + PAIRS_PER_GPU
 
-    def run_steps(submit, K):
+    region = {}
+
+    def run_steps(submit, K, lead=0, tail=0):
+        """`lead` untimed steps, K timed steps and `tail` untimed steps back to back.  Returns the host seconds from the
+        completion of the last lead step (from the call when lead == 0) to the completion of the last timed step, plus the
+        exchange of the timed steps' records.  With lead >= DEPTH and tail == DEPTH - 1 the pipeline is full from the start to
+        the end of that window, so it measures K steps of steady state."""
         if comm is not None:
             pin = local_edges["pin_buf"]
             local_edges["buf"] = pin[1][:K * PAIRS_PER_GPU] if pin is not None and len(pin[1]) >= K * PAIRS_PER_GPU else \
                 np.zeros(K * PAIRS_PER_GPU, PAIR_RESULT_DTYPE)
             local_edges["n"] = 0
-        for k in range(K):
+        n = lead + K + tail
+        t = {"start": time.perf_counter()}
+
+        def done(j):
+            finish(j, lead <= j < lead + K)
+            if j == lead - 1:
+                t["start"] = time.perf_counter()
+            elif j == lead + K - 1:
+                t["end"] = time.perf_counter()
+                last = sets[j % DEPTH]  # what the last timed step handed to its caller
+                region["last"] = {k: last[k].copy() for k in ("res", "allm", "inl")}
+
+        for k in range(n):
             if k >= DEPTH:
-                finish(k - DEPTH)
+                done(k - DEPTH)
+            if k == lead:
+                launches0 = fe.launch_count
+            elif k == lead + K:
+                region["launches"] = fe.launch_count - launches0
             submit(k)
-        for k in range(max(0, K - DEPTH), K):
-            finish(k)
+        if tail == 0:
+            region["launches"] = fe.launch_count - launches0
+        for j in range(max(0, n - DEPTH), n):
+            done(j)
+        dt = t["end"] - t["start"]
         if comm is not None:  # the one exchange: every rank ends up with every rank's edges of the whole region
+            t0 = time.perf_counter()
             pin = local_edges["pin_all"]
             out = pin[1][:world * K * PAIRS_PER_GPU] if pin is not None and len(pin[1]) >= world * K * PAIRS_PER_GPU else None
             local_edges["all"] = fe.allgather_edges(comm, local_edges["buf"], world, out=out)
+            dt += time.perf_counter() - t0
+        return dt
 
     def barrier():
         torch.cuda.synchronize()
@@ -737,39 +769,21 @@ def run_ours(args, rank, local_rank, world):
         sampler.start()
 
     # ---- timed: device-resident inputs, pipelined over DEPTH slots ------------------------------------
-    # --steps K is timed as R back-to-back blocks of K steps so that the region covers >= MIN_TIMED_MS (20 steps of 0.15 ms
-    # are four pipeline turn-overs); per-step numbers divide by K * R.  R comes from a short probe, identical on every rank.
-    run_steps(submit_resident, max(args.steps, DEPTH))  # first region of this size: the exchange buffers are allocated here
-    torch.cuda.synchronize()
-    p0 = time.perf_counter()
-    run_steps(submit_resident, max(args.steps, DEPTH))
-    torch.cuda.synchronize()
-    probe = torch.tensor([(time.perf_counter() - p0) / max(args.steps, DEPTH)], dtype=torch.float64, device="cuda")
-    if world > 1:
-        dist.all_reduce(probe, op=dist.ReduceOp.MAX)
-    # a short probe region over-estimates the step (pipeline ramp, the exchange): never fewer steps than MIN_TIMED_MS of the
-    # fastest step this code has measured (0.12 ms), or the fixed costs of a region dominate it (the first 2- and 8-GPU lines of
-    # round 2 timed 6 and 41 ms)
-    repeats = max(1, int(np.ceil(MIN_TIMED_MS * 1e-3 / (float(probe.item()) * args.steps))),
-                  int(np.ceil(MIN_TIMED_MS / (0.12 * args.steps))))
-    timed_steps = args.steps * repeats
+    # exactly --steps K steps between DEPTH untimed steps that fill the pipeline and DEPTH - 1 that keep it full, so that a short
+    # region measures neither the ramp nor the drain (20 steps of 0.15 ms are four pipeline turn-overs).  The host clock reads
+    # after the stream synchronise of a step.
+    timed_steps = args.steps
     reserve_exchange(timed_steps)
-    launches0 = fe.launch_count
-    ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
-    wall0 = time.perf_counter()
-    ev0.record(stream)
-    run_steps(submit_resident, timed_steps)
-    torch.cuda.synchronize()
-    ev1.record(stream)
+    resident_s = run_steps(submit_resident, timed_steps, lead=DEPTH, tail=DEPTH - 1)
     barrier()
-    wall_resident = time.perf_counter() - wall0
-    launches = fe.launch_count - launches0
+    launches = region["launches"]
+    resident_out = region["last"]["res"]
     ham_ms, dev_ms = [], []
     for j in range(DEPTH):
         h, t = fe.last_timing(1 + j)
         ham_ms.append(h); dev_ms.append(t)
-    total_ms = torch.tensor([ev0.elapsed_time(ev1)], dtype=torch.float64, device="cuda")
+    total_ms = torch.tensor([1e3 * resident_s], dtype=torch.float64, device="cuda")
     if world > 1:
         dist.all_reduce(total_ms, op=dist.ReduceOp.MAX)
     total_ms = float(total_ms.item())
@@ -777,11 +791,14 @@ def run_ours(args, rank, local_rank, world):
 
     # ---- timed: end to end through the host-buffer C ABI (pinned host buffers in, host results out) -----
     barrier()
-    t0 = time.perf_counter()
-    run_steps(submit_e2e, timed_steps)
-    torch.cuda.synchronize()
-    e2e_wall = time.perf_counter() - t0
+    e2e_wall = run_steps(submit_e2e, timed_steps, lead=DEPTH, tail=DEPTH - 1)
     barrier()
+    e2e_out = region["last"]
+    if rank == 0 and args.dump_outputs is not None:
+        dump_outputs(args.dump_outputs, {
+            "resident_results": resident_out, "e2e_results": e2e_out["res"],
+            "e2e_all_matches": first_n(e2e_out["allm"], e2e_out["res"]["n_all_matches"]),
+            "e2e_inlier_matches": first_n(e2e_out["inl"], e2e_out["res"]["n_inliers"])})
     e2e_total = torch.tensor([e2e_wall], dtype=torch.float64, device="cuda")
     if world > 1:
         dist.all_reduce(e2e_total, op=dist.ReduceOp.MAX)
@@ -836,8 +853,10 @@ def run_ours(args, rank, local_rank, world):
                        "pairs_per_gpu": PAIRS_PER_GPU,
                        "exchange": "none (1 GPU)" if world == 1 else f"ONE ncclAllGather of the {world} x {timed_steps} x {PAIRS_PER_GPU} edge records (120 B) of the region at its end (rgbdslam_b200_allgather_edges), inside the timed region",
                        "edges_gathered": None if comm is None else int((local_edges["all"]["id1"] >= 0).sum()),
-                       "valid_edges_rank0": n_valid, "wall_ms_per_step_incl_flush": 1e3 * wall_resident / timed_steps,
-                       "repeats": f"{repeats} x --steps {args.steps} timed back to back (>= {MIN_TIMED_MS:.0f} ms per timed region)"},
+                       "valid_edges_rank0": n_valid,
+                       "timing": f"--steps {args.steps} timed back to back between {DEPTH} untimed steps that fill the pipeline "
+                                 f"and {DEPTH - 1} that keep it full; host clock from the completion of the step before the first "
+                                 "timed step to that of the last timed step"},
             "roofline": {"bound": "hbm", "kernel": "hamming_match", "achieved": achieved, "peak": peak, "unit": "GB/s",
                          "frac": achieved / peak, "traffic": NCU_DRAM_BYTES_PER_LAUNCH, "traffic_source": NCU_TRAFFIC_SOURCE, "peak_source": peak_src,
                          "algorithmic_bytes_per_launch": ALGO_BYTES_PER_PAIR * PAIRS_PER_GPU, "kernel_ms": ham,
@@ -904,6 +923,23 @@ def run_ours(args, rank, local_rank, world):
         dist.destroy_process_group()
 
 
+def first_n(matches: np.ndarray, n: np.ndarray) -> np.ndarray:
+    """Row i keeps its first n[i] entries, the rest are zeroed: only those were written by the step."""
+    out = matches.copy()
+    out[np.arange(matches.shape[1])[None, :] >= n[:, None]] = np.zeros(1, matches.dtype)
+    return out
+
+
+def dump_outputs(d: Path, arrays: dict):
+    """One DIR/<name>_<field>.npy per field of each structured array: float32 fields as they are, every other field as
+    float64 (exact for these 32-bit integers).  Padding fields (trailing underscore) are left out."""
+    d.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        for f in a.dtype.names:
+            if not f.endswith("_"):
+                np.save(d / f"{name}_{f}.npy", a[f].astype(np.float32 if a[f].dtype == np.float32 else np.float64))
+
+
 _JSON_OUT = None
 
 
@@ -923,7 +959,13 @@ def main():
     ap.add_argument("--no-c4", action="store_true", help="skip the 2000-frame sequence (config C4) sub-measurement")
     ap.add_argument("--c4-frames", type=int, default=C4_FRAMES)
     ap.add_argument("--no-c3", action="store_true", help="skip the SIFT-128 (config C3) sub-measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", type=Path,
+                    help="write the results of the last timed step as DIR/<name>.npy (--impl ours)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

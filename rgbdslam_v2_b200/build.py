@@ -38,18 +38,22 @@ def build_library(force: bool = False, verbose: bool = False) -> Path:
     """Compile csrc/*.cu into librgbdslam_b200.so (skipped if up to date)."""
     import fcntl
     out = PKG_DIR / LIB_NAME
+    if not force and _up_to_date(out):  # nothing is written then: the tree may be read-only once built
+        return out
     with open(PKG_DIR / ".build.lock", "w") as lk:  # several ranks may call build() at once
         fcntl.flock(lk, fcntl.LOCK_EX)
         return _build_locked(out, force, verbose)
 
 
+def _up_to_date(out: Path) -> bool:
+    deps = sources() + sorted(CSRC.glob("*.h")) + sorted(CSRC.glob("*.cuh")) + [PKG_DIR.parent / "include" / "rgbdslam_b200.h"]
+    return out.exists() and out.stat().st_mtime >= max(p.stat().st_mtime for p in deps)
+
+
 def _build_locked(out: Path, force: bool, verbose: bool) -> Path:
+    if not force and _up_to_date(out):
+        return out
     srcs = sources()
-    deps = srcs + sorted(CSRC.glob("*.h")) + sorted(CSRC.glob("*.cuh")) + [PKG_DIR.parent / "include" / "rgbdslam_b200.h"]
-    if out.exists() and not force:
-        newest = max(p.stat().st_mtime for p in deps)
-        if out.stat().st_mtime >= newest:
-            return out
     cmd = [_nvcc(), *NVCC_FLAGS, "-o", str(out), *map(str, srcs)]
     if verbose:
         cmd.insert(1, "-Xptxas=-v")
